@@ -1,6 +1,7 @@
 """bench.py -- env steps/sec of a batched random-policy Crafter rollout on N B200s (BASELINE.json).
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME]
+                    [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one tick of every env of the batch.  `--config default` is BASELINE.json configs[1]
@@ -196,6 +197,27 @@ def regime_block(before, after, steps):
   return out
 
 
+DUMP_BYTES = 60 * 10 ** 6  # what --dump-outputs writes in all stays below 64 MB, .npy headers included
+
+
+def dump_outputs(directory, obs, reward, done, info):
+  """What the last timed step returned, as float32 DIR/<name>.npy (every value is a small integer or a
+  reward, so exactly): reward, done, inventory, achievements and player_pos of every env, and obs of
+  every env when they fit, else of a fixed sample of envs (np.random.RandomState(0), ascending)."""
+  import numpy as np
+  import torch
+  out = pathlib.Path(directory)
+  out.mkdir(parents=True, exist_ok=True)
+  arrays = dict(reward=reward, done=done, inventory=info['inventory'], achievements=info['achievements'],
+                player_pos=info['player_pos'])
+  B = obs.shape[0]
+  n = min(B, (DUMP_BYTES - 4 * sum(a.numel() for a in arrays.values())) // (4 * obs[0].numel()))
+  rows = np.sort(np.random.RandomState(0).choice(B, n, replace=False)) if n < B else np.arange(B)
+  arrays['obs'] = obs[torch.as_tensor(rows, device=obs.device)]
+  for name, a in arrays.items():
+    np.save(out / f'{name}.npy', a.cpu().numpy().astype(np.float32))
+
+
 def kernel_times(kwargs, seed, rank_offset, state_dict, actions, steps):
   """Per-kernel device durations INSIDE the step graph: a second handle created with
   CRAFTER_B200_TIMING=2 (event-record nodes around every kernel of the captured graph), loaded with
@@ -233,7 +255,13 @@ def main():
   ap.add_argument('--config', default='default', choices=sorted(CONFIGS))
   ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
   ap.add_argument('--no-cpu-baseline', action='store_true')
+  ap.add_argument('--dump-outputs', metavar='DIR',
+                  help='write what the last timed step returned (rank 0) as DIR/<name>.npy, see dump_outputs')
   args = ap.parse_args()
+  if args.steps < 1:
+    ap.error('--steps must be at least 1')
+  if args.dump_outputs and args.impl != 'ours':
+    ap.error('--dump-outputs writes what the CUDA path returned; it needs --impl ours')
   args.warmup = max(args.warmup, 3)
   rank = int(os.environ.get('RANK', 0))
   local_rank = int(os.environ.get('LOCAL_RANK', 0))
@@ -286,11 +314,13 @@ def main():
     flush.zero_()
     stream.wait_stream(torch.cuda.current_stream(device))
     starts[k].record(stream)
-    env.step(env.actions_buffer)
+    last = env.step(env.actions_buffer)
     ends[k].record(stream)
   barrier()
   wall = time.perf_counter() - wall0
   clocks = sampler.stop()
+  if args.dump_outputs and rank == 0:  # before the legs below step the env on
+    dump_outputs(args.dump_outputs, *last)
   launches = env.launch_count - launches0
   probe1 = regime_probe(env)
   step_ms = [s.elapsed_time(e) for s, e in zip(starts, ends)]

@@ -39,7 +39,7 @@ PSTATE = ['hunger2', 'thirst2', 'fatigue', 'recover2', 'sleeping', 'player_last_
           'player_y', 'error', 'episode_length']
 
 # The numeric rule tables (data.yaml:34-78), restated for documentation and for the tests that (a) diff
-# them against the reference's data.yaml when it is mounted and (b) probe the device code
+# them against the reference's data.yaml (tests/golden/data_yaml.json) and (b) probe the device code
 # (csrc/cr_update.h player_do_material / player_place / player_make, csrc/cr_worldgen.h wg_fresh_player)
 # with them, entry by entry (tests/test_rules_table.py).
 WALKABLE = ['grass', 'sand', 'path']

@@ -1,6 +1,6 @@
-"""TEST INFRASTRUCTURE shared by the live scenario fuzz (tests/test_scenarios_vs_reference.py, build
-container only), the fixture generator (tools/make_scenarios.py) and the fixture replay
-(tests/test_scenarios_golden.py: host-sim on CPU, the CUDA library on the GPU box).
+"""TEST INFRASTRUCTURE shared by the fixture generator (tools/make_scenarios.py) and the fixture replays
+(tests/test_scenarios_golden.py: host-sim on CPU, the CUDA library on the GPU box;
+tests/test_scenarios_vs_reference.py: the perturbation fuzz on the host-sim).
 
 A *scenario* is a state that random rollouts rarely reach, built INSIDE a live reference env through
 the reference's own World / object API (engine.py, objects.py), exported as a canonical state
@@ -69,8 +69,36 @@ def load_torch(state, i, raw):
     state[k][i].copy_(torch.from_numpy(np.ascontiguousarray(v)))
 
 
-def extras_of(env):
-  return dict(step=int(env._step), episode=int(env._episode), world_seed=int(env._world.random.seed))
+# ---- packed fixture layout -----------------------------------------------------------------------
+def pack(blob):
+  """A fixture's s{i}_{key} members as one member per key: p_{key} (the arrays of every scenario,
+  flattened and concatenated) and p_{key}_shapes (K, ndim).  Far fewer .npz members, and they
+  compress better than one small member per scenario and key."""
+  out, parts = {}, {}
+  for k, v in blob.items():
+    if k.startswith('meta_'):
+      out[k] = v
+    else:
+      i, key = k[1:].split('_', 1)
+      parts.setdefault(key, {})[int(i)] = np.asarray(v)
+  for key, by_index in parts.items():
+    arrays = [by_index[i] for i in range(len(by_index))]
+    out[f'p_{key}'] = np.concatenate([a.reshape(-1) for a in arrays])
+    out[f'p_{key}_shapes'] = np.array([a.shape for a in arrays], np.int64).reshape(len(arrays), arrays[0].ndim)
+  return out
+
+
+def unpack(z):
+  """Inverse of pack: a dict with the s{i}_{key} members of the unpacked layout."""
+  out = {k: z[k] for k in z.files if k.startswith('meta_')}
+  for k in z.files:
+    if k.startswith('p_') and not k.endswith('_shapes'):
+      flat, at = z[k], 0
+      for i, shape in enumerate(z[k + '_shapes']):
+        n = int(np.prod(shape))
+        out[f's{i}_{k[2:]}'] = flat[at:at + n].reshape(shape)
+        at += n
+  return out
 
 
 # ---- helpers over the reference's API -------------------------------------------------------------

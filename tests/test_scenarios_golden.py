@@ -24,8 +24,9 @@ def to_numpy(x):
   return x.detach().cpu().numpy() if hasattr(x, 'detach') else np.asarray(x)
 
 
-def replay_group(group, make_env, load):
-  z = np.load(SCEN / f'{group}.npz')
+def replay_group(group, make_env, load, z=None):
+  """z: the fixture's members (default: tests/golden/scenarios/<group>.npz)."""
+  z = np.load(SCEN / f'{group}.npz') if z is None else z
   K = int(z['meta_K'])
   names = [str(n) for n in z['meta_names']]
   kwargs = dict(area=tuple(int(v) for v in z['meta_area']), view=tuple(int(v) for v in z['meta_view']),

@@ -8,7 +8,8 @@ of the canonical state, reward, done and the observation digest -- all produced 
 under oracle/ref_harness.py.  tests/test_scenarios_golden.py replays them through the host-sim on
 CPU and through the CUDA library (C ABI) on the GPU box.
 
-    python tools/make_scenarios.py            # writes every group in GROUPS
+    python tools/make_scenarios.py            # writes every group in GROUPS and PERTURBED
+    python tools/make_scenarios.py perturbed  # only tests/golden/perturbed/
 """
 import pathlib
 import sys
@@ -33,6 +34,12 @@ GROUPS = {
     'directed_short': (dict(length=300, area=(48, 56), view=(7, 9), size=(70, 72)), 'directed', None, 4000),
 }
 FUZZ_STEPS = 45
+# The perturbation stream tests/test_scenarios_vs_reference.py replays from tests/golden/perturbed/
+# (random stream 4711, world seeds 5000 + round): name -> (env kwargs, rounds, steps per round)
+PERTURBED = {
+    'default': (dict(), 40, 45),
+    'small': (dict(area=(24, 20)), 30, 40),
+}
 
 
 def record(env, actions):
@@ -68,16 +75,16 @@ def record(env, actions):
   return out
 
 
-def build(kwargs, kind, count, seed0):
+def build(kwargs, kind, count, seed0, stream=2024, steps=FUZZ_STEPS):
   mods = rh.load()
   scenarios, names = [], []
   if kind == 'fuzz':
-    rs = np.random.RandomState(2024)
+    rs = np.random.RandomState(stream)
     for r in range(count):
       env = rh.make_env(seed0 + r, **kwargs)
       env.reset()
       su.perturb(env, rs, mods)
-      scenarios.append(record(env, su.fuzz_actions(rs, FUZZ_STEPS)))
+      scenarios.append(record(env, su.fuzz_actions(rs, steps)))
       names.append(f'fuzz{r}')
   else:
     for r, (name, fn) in enumerate(su.DIRECTED):
@@ -91,27 +98,36 @@ def build(kwargs, kind, count, seed0):
 
 
 def main(groups):
-  outdir = ROOT / 'tests' / 'golden' / 'scenarios'
-  outdir.mkdir(parents=True, exist_ok=True)
   for g in groups:
-    kwargs, kind, count, seed0 = GROUPS[g]
-    names, scenarios = build(kwargs, kind, count, seed0)
-    blob = dict(
-        meta_area=np.array(kwargs.get('area', (64, 64))), meta_view=np.array(kwargs.get('view', (9, 9))),
-        meta_size=np.array(kwargs.get('size', (64, 64))), meta_length=np.array(kwargs.get('length', 10000)),
-        meta_seed0=np.array(seed0), meta_K=np.array(len(scenarios)), meta_names=np.array(names))
-    ach, steps, deaths = 0, 0, 0
-    for i, s in enumerate(scenarios):
-      for k, v in s.items():
-        blob[f's{i}_{k}'] = v
-      ach |= int(s['player_t'][:, 16:38].max(0).astype(bool) @ (1 << np.arange(22)))
-      steps += len(s['actions'])
-      deaths += int(s['done'].any())
-    path = outdir / f'{g}.npz'
-    np.savez_compressed(path, **blob)
-    print(f'{g}: {len(scenarios)} scenarios, {steps} steps, {deaths} ended, '
-          f'{bin(ach).count("1")}/22 achievements touched, {path.stat().st_size / 1024:.0f} KiB')
+    if g == 'perturbed':
+      for name, (kwargs, count, steps) in PERTURBED.items():
+        names, scenarios = build(kwargs, 'fuzz', count, 5000, stream=4711, steps=steps)
+        for s in scenarios:
+          del s['obs_last']  # no replay reads it, and it would be half of the file
+        save(ROOT / 'tests' / 'golden' / 'perturbed' / f'{name}.npz', kwargs, 5000, names, scenarios, packed=True)
+    else:
+      kwargs, kind, count, seed0 = GROUPS[g]
+      names, scenarios = build(kwargs, kind, count, seed0)
+      save(ROOT / 'tests' / 'golden' / 'scenarios' / f'{g}.npz', kwargs, seed0, names, scenarios)
+
+
+def save(path, kwargs, seed0, names, scenarios, packed=False):
+  blob = dict(
+      meta_area=np.array(kwargs.get('area', (64, 64))), meta_view=np.array(kwargs.get('view', (9, 9))),
+      meta_size=np.array(kwargs.get('size', (64, 64))), meta_length=np.array(kwargs.get('length', 10000)),
+      meta_seed0=np.array(seed0), meta_K=np.array(len(scenarios)), meta_names=np.array(names))
+  ach, steps, deaths = 0, 0, 0
+  for i, s in enumerate(scenarios):
+    for k, v in s.items():
+      blob[f's{i}_{k}'] = v
+    ach |= int(s['player_t'][:, 16:38].max(0).astype(bool) @ (1 << np.arange(22)))
+    steps += len(s['actions'])
+    deaths += int(s['done'].any())
+  path.parent.mkdir(parents=True, exist_ok=True)
+  np.savez_compressed(path, **(su.pack(blob) if packed else blob))
+  print(f'{path.stem}: {len(scenarios)} scenarios, {steps} steps, {deaths} ended, '
+        f'{bin(ach).count("1")}/22 achievements touched, {path.stat().st_size / 1024:.0f} KiB')
 
 
 if __name__ == '__main__':
-  main(sys.argv[1:] or list(GROUPS))
+  main(sys.argv[1:] or list(GROUPS) + ['perturbed'])
