@@ -68,7 +68,7 @@ CR_DEV double noise_extrapolate(const NoiseTables &t, int xsb, int ysb, int zsb,
 //     lattice offset o,   displacement ((d0 - A) - k * SQUISH) - C      per axis, per extra vertex
 // with A in {-1,0,1,2}, k in {0..3}, C in {0,1,2} and o = A + C (the published code writes e.g.
 // `dy0 - 1 - 3*SQ` and later `-= 1`: A=1, k=3, C=1; subtracting a zero is exact).  A warp would
-// otherwise execute the union of all leaves; here the branches only pick a case number and the
+// otherwise execute the union of all leaves; here the region tests only pick a case number and the
 // leaf is data: noise_ext_case(id) packs it into 6 bytes, staged once per CTA in shared memory.
 // byte of (extra vertex e, axis a) at bits 8 * (3 * e + a): (A + 1) | k << 2 | C << 4
 CR_DEV uint64_t noise_ext_pack(const int (&A)[2][3], const int (&K)[2][3], const int (&C)[2][3]) {
@@ -171,51 +171,42 @@ CR_DEV double noise3(const NoiseTables &t, double x, double y, double z, int *ca
 
   unsigned member;  // bit v set: cube vertex v of the sequence above contributes
   int id;           // which of the 27 extra-vertex assignments
-  if (in_sum <= 1) {  // tetrahedron at (0,0,0)
-    member = 0x0Fu;
-    int a_point = 0x01, b_point = 0x02;
-    double a_score = xins, b_score = yins;
-    if (a_score >= b_score && zins > b_score) { b_score = zins; b_point = 0x04; }
-    else if (a_score < b_score && zins > a_score) { a_score = zins; a_point = 0x04; }
-    double wins = 1 - in_sum;
-    if (wins > a_score || wins > b_score) id = noise_bit((b_score > a_score) ? b_point : a_point);
-    else id = 3 + noise_bit(7 ^ (a_point | b_point));
-  } else if (in_sum >= 2) {  // tetrahedron at (1,1,1)
-    member = 0xF0u;
-    int a_point = 0x06, b_point = 0x05;
-    double a_score = xins, b_score = yins;
-    if (a_score <= b_score && zins < b_score) { b_score = zins; b_point = 0x03; }
-    else if (a_score > b_score && zins < a_score) { a_score = zins; a_point = 0x03; }
-    double wins = 3 - in_sum;
-    if (wins < a_score || wins < b_score) id = 6 + noise_bit(7 ^ ((b_score < a_score) ? b_point : a_point));
-    else id = 9 + noise_bit(a_point & b_point);
-  } else {  // octahedron in between
-    member = 0x7Eu;
-    double a_score, b_score;
-    int a_point, b_point;
-    bool a_far, b_far;
-    double p1 = xins + yins;
-    if (p1 > 1) { a_score = p1 - 1; a_point = 0x03; a_far = true; }
-    else { a_score = 1 - p1; a_point = 0x04; a_far = false; }
-    double p2 = xins + zins;
-    if (p2 > 1) { b_score = p2 - 1; b_point = 0x05; b_far = true; }
-    else { b_score = 1 - p2; b_point = 0x02; b_far = false; }
-    double p3 = yins + zins;
-    if (p3 > 1) {
-      double score = p3 - 1;
-      if (a_score <= b_score && a_score < score) { a_point = 0x06; a_far = true; }
-      else if (a_score > b_score && b_score < score) { b_point = 0x06; b_far = true; }
-    } else {
-      double score = 1 - p3;
-      if (a_score <= b_score && a_score < score) { a_point = 0x01; a_far = false; }
-      else if (a_score > b_score && b_score < score) { b_point = 0x01; b_far = false; }
-    }
-    if (a_far == b_far) {
-      id = a_far ? 12 + noise_bit(a_point & b_point) : 15 + noise_bit(7 ^ (a_point | b_point));
-    } else {
-      const int c1 = a_far ? a_point : b_point, c2 = a_far ? b_point : a_point;
-      id = 18 + 3 * noise_bit(7 ^ c1) + noise_bit(c2);
-    }
+  // All three regions' tests are evaluated and the region picks among the results: a warp holds
+  // lanes of all three regions almost always, so branches would run all three blocks anyway.  Each
+  // test compares the same doubles with the same relation as the published branches.
+  {  // tetrahedron at (0,0,0)
+    const bool b_z = xins >= yins && zins > yins, a_z = xins < yins && zins > xins;
+    const double a_score = a_z ? zins : xins, b_score = b_z ? zins : yins;
+    const int a_point = a_z ? 0x04 : 0x01, b_point = b_z ? 0x04 : 0x02;
+    const double wins = 1 - in_sum;
+    const int near = noise_bit((b_score > a_score) ? b_point : a_point);
+    id = (wins > a_score || wins > b_score) ? near : 3 + noise_bit(7 ^ (a_point | b_point));
+  }
+  {  // tetrahedron at (1,1,1)
+    const bool b_z = xins <= yins && zins < yins, a_z = xins > yins && zins < xins;
+    const double a_score = a_z ? zins : xins, b_score = b_z ? zins : yins;
+    const int a_point = a_z ? 0x03 : 0x06, b_point = b_z ? 0x03 : 0x05;
+    const double wins = 3 - in_sum;
+    const int near = 6 + noise_bit(7 ^ ((b_score < a_score) ? b_point : a_point));
+    const int id_far = (wins < a_score || wins < b_score) ? near : 9 + noise_bit(a_point & b_point);
+    id = in_sum <= 1 ? id : id_far;
+  }
+  {  // octahedron in between
+    const double p1 = xins + yins, p2 = xins + zins, p3 = yins + zins;
+    const bool a_far0 = p1 > 1, b_far0 = p2 > 1, far3 = p3 > 1;
+    const double a_score = a_far0 ? p1 - 1 : 1 - p1, b_score = b_far0 ? p2 - 1 : 1 - p2;
+    const double score = far3 ? p3 - 1 : 1 - p3;
+    const bool to_a = a_score <= b_score && a_score < score, to_b = a_score > b_score && b_score < score;
+    const int p3_point = far3 ? 0x06 : 0x01;
+    const int a_point = to_a ? p3_point : (a_far0 ? 0x03 : 0x04);
+    const int b_point = to_b ? p3_point : (b_far0 ? 0x05 : 0x02);
+    const bool a_far = to_a ? far3 : a_far0, b_far = to_b ? far3 : b_far0;
+    const int c1 = a_far ? a_point : b_point, c2 = a_far ? b_point : a_point;
+    const int id_same = a_far ? 12 + noise_bit(a_point & b_point) : 15 + noise_bit(7 ^ (a_point | b_point));
+    const int id_oct = a_far == b_far ? id_same : 18 + 3 * noise_bit(7 ^ c1) + noise_bit(c2);
+    const bool oct = !(in_sum <= 1) && !(in_sum >= 2);
+    id = oct ? id_oct : id;
+    member = in_sum <= 1 ? 0x0Fu : in_sum >= 2 ? 0xF0u : 0x7Eu;
   }
 
   // the leaf as data: lattice offsets and displacements of the two extra vertices

@@ -117,11 +117,11 @@ CR_DEV int wg_object(const Geom &g, uint32_t world_seed, int x, int y, uint8_t m
 
 // ---- terrain: worldgen.py:21-61, a tile of cells per CTA, octaves evaluated from a work list ----
 // The reference evaluates up to 11 simplex octaves per cell, lazily, one after another; which ones
-// depends on the cell.  Here a CTA owns WG_TILE cells and proceeds in at most five rounds; in each
+// depends on the cell.  Here a CTA owns WG_TILE cells and proceeds in at most four rounds; in each
 // round every unfinished cell posts the octaves its current phase needs, the (cell, octave) items
 // are processed densely by all threads through ONE noise3 call site, and a per-cell combine step
 // applies the reference's branches (with its uniform draws, in its order) and picks the next phase.
-// Only the tunnel / ore octaves are evaluated eagerly together.  Otherwise a cell evaluates a SUBSET of
+// The start, water and mountain octaves are evaluated together, and so are the tunnel / ore octaves.  Otherwise a cell evaluates a SUBSET of
 // the reference's lazy set: an octave whose threshold test is and-ed with a condition that is already
 // known to fail (`simplex(..) > 0 and uniform() > 0.8`, `simplex(..) > 0.15 and mountain > 0.3`) cannot
 // change the cell, and the keyed draws do not depend on the order they are looked at -- so the cheap
@@ -131,22 +131,59 @@ CR_DEV int wg_object(const Geom &g, uint32_t world_seed, int x, int y, uint8_t m
 #endif
 constexpr int WG_TILE = CR_WG_TILE;
 constexpr int WG_N_OCTAVES = 28;  // phase * 4 + slot
-enum WgPhase : int8_t { WP_DONE = -1, WP_START = 0, WP_WM, WP_CAVE, WP_SAND, WP_TREE, WP_TUNNEL, WP_LAVA };
+// WP_START posts five octaves at once (slots 0-3 water / mountain, slot 4 start: octave codes 0..4),
+// so a cell goes through at most four rounds: START, CAVE, TUNNEL, LAVA.  Only cells within a few
+// cells of the map centre (start > 0.5, ~3 % of a 64 x 64 map) have no use for the four water /
+// mountain values; evaluating them costs less than a round of its own.
+enum WgPhase : int8_t { WP_DONE = -1, WP_START = 0, WP_CAVE = 2, WP_SAND, WP_TREE, WP_TUNNEL, WP_LAVA };
+constexpr int WG_ROUNDS = 4, WG_SLOTS = 5;
+
+enum WgOctaveKind { WO_PLAIN = 0, WO_TUNNEL_H = 1, WO_TUNNEL_V = 2 };
+
+// a / d for r = 1 / d: the product's error is removed with the exact remainder (Markstein).  This is
+// the correctly rounded quotient -- the same double as `a / d` -- for every a a map side < 32768 makes
+// (x or 2x over d in {3, 5, 6, 7, 8, 9, 15}, x / 5 over 3; all checked by tests/test_noise_boundaries.py),
+// in three FP64 instructions where `/` takes a reciprocal, Newton steps and a range check.
+CR_DEV double wg_div(double a, double d, double r) {
+  const double q = a * r;
+  return fma(fma(-q, d, a), r, q);
+}
+
+// An octave's arguments as data: per axis the numerator's factor and the divisor with its reciprocal;
+// `again` = 1 / 2: the x / y quotient is divided by 3 once more (the tunnel octaves).
+struct WgOctave {
+  double dx, rx, dy, ry, z;
+  int mx, my, again;
+};
+
+CR_DEV WgOctave wg_octave(uint32_t code) {
+  const int size = code & 15, kind = code >> 8;
+  WgOctave o;
+  o.mx = kind == WO_TUNNEL_H ? 2 : 1;
+  o.my = kind == WO_TUNNEL_V ? 2 : 1;
+  o.dx = kind == WO_TUNNEL_V ? 5.0 : (double)size;
+  o.dy = kind == WO_TUNNEL_H ? 5.0 : (double)size;
+  o.rx = 1 / o.dx;
+  o.ry = 1 / o.dy;
+  o.z = (double)((code >> 4) & 15);
+  o.again = kind == WO_TUNNEL_V ? 1 : kind == WO_TUNNEL_H ? 2 : 0;
+  return o;
+}
 
 struct WgTile {  // shared memory of one CTA
   double start[WG_TILE], water[WG_TILE], mountain[WG_TILE];
   double v[WG_TILE][4];
-  uint16_t items[WG_TILE * 4];  // cell * 4 + slot
+  uint16_t items[WG_TILE * WG_SLOTS];  // cell * 8 + slot
   int32_t n_items;
   int8_t phase[WG_TILE];
   uint8_t need[WG_TILE];    // WP_TUNNEL: which of the four octaves can still change the cell (bit = slot)
   uint8_t result[WG_TILE];
-  uint16_t oct[WG_N_OCTAVES];  // wg_octave_code
+  WgOctave oct[WG_N_OCTAVES];  // wg_octave(wg_octave_code(i))
 };
 
 // octaves (bit = slot) a cell in `phase` posts
 CR_DEV unsigned wg_phase_slots(int phase, unsigned need) {
-  return phase == WP_WM ? 0xFu : phase == WP_TUNNEL ? need : 1u;
+  return phase == WP_START ? 0x1Fu : phase == WP_TUNNEL ? need : 1u;
 }
 
 // worldgen.py:49-58 below the two tunnel tests, as a function of the two ore thresholds
@@ -188,19 +225,18 @@ CR_DEV int wg_enter_tree(const Geom &g, uint32_t world_seed, int x, int y) {
 
 // _simplex(x, y, z, size) -> noise3(x / size, y / size, z) for the octave (phase, slot) asks for
 // (worldgen.py:27-60,79-91).  The items of a warp ask for different octaves, so the octave is data
-// (wg_octave_code, staged once per CTA as T.oct[]) and every lane runs the same two divisions;
-// only the tunnel octaves `(2x, y/5, 7, 3)` / `(x/5, 2y, 7, 3)` pay a second one.
-enum WgOctaveKind { WO_PLAIN = 0, WO_TUNNEL_H = 1, WO_TUNNEL_V = 2 };
-
+// (wg_octave_code -> wg_octave, staged once per CTA as T.oct[]) and every lane runs the same
+// divisions: one per axis, and a third that only the tunnel octaves `(2x, y/5, 7, 3)` /
+// `(x/5, 2y, 7, 3)` keep.
 // size | z << 4 | kind << 8
 CR_DEV uint16_t wg_octave_code(int code) {
   int size = 5, z = 6, kind = WO_PLAIN;                               // lava     (x, y, 6, 5)
   switch (code) {
-    case WP_START * 4: size = 3; z = 8; break;                        // start    (x, y, 8, 3)
-    case WP_WM * 4 + 0: size = 15; z = 3; break;                      // water    (x, y, 3, 15)
-    case WP_WM * 4 + 1: size = 5; z = 3; break;                       // water    (x, y, 3, 5)
-    case WP_WM * 4 + 2: size = 15; z = 0; break;                      // mountain (x, y, 0, 15)
-    case WP_WM * 4 + 3: size = 5; z = 0; break;                       // mountain (x, y, 0, 5)
+    case WP_START * 4 + 0: size = 15; z = 3; break;                   // water    (x, y, 3, 15)
+    case WP_START * 4 + 1: size = 5; z = 3; break;                    // water    (x, y, 3, 5)
+    case WP_START * 4 + 2: size = 15; z = 0; break;                   // mountain (x, y, 0, 15)
+    case WP_START * 4 + 3: size = 5; z = 0; break;                    // mountain (x, y, 0, 5)
+    case WP_START * 4 + 4: size = 3; z = 8; break;                    // start    (x, y, 8, 3)
     case WP_CAVE * 4: size = 7; z = 6; break;                         // cave     (x, y, 6, 7)
     case WP_SAND * 4: size = 9; z = 4; break;                         // sand     (x, y, 4, 9)
     case WP_TREE * 4: size = 7; z = 5; break;                         // tree     (x, y, 5, 7)
@@ -213,16 +249,30 @@ CR_DEV uint16_t wg_octave_code(int code) {
   return (uint16_t)(size | (z << 4) | (kind << 8));
 }
 
-CR_DEV void wg_octave_args(uint32_t oct, int x, int y, double &ax, double &ay, double &az) {
-  const int size = oct & 15, kind = oct >> 8;
-  const double fsize = (double)size;
-  // plain: x / size.   tunnel-h: (2x) / 3, (y / 5) / 3.   tunnel-v: (x / 5) / 3, (2y) / 3.
-  const double nx = (double)(kind == WO_TUNNEL_H ? 2 * x : x), ny = (double)(kind == WO_TUNNEL_V ? 2 * y : y);
-  ax = nx / (kind == WO_TUNNEL_V ? 5.0 : fsize);
-  ay = ny / (kind == WO_TUNNEL_H ? 5.0 : fsize);
-  if (kind == WO_TUNNEL_V) ax = ax / 3;
-  if (kind == WO_TUNNEL_H) ay = ay / 3;
-  az = (double)((oct >> 4) & 15);
+CR_DEV void wg_octave_args(const WgOctave &o, int x, int y, double &ax, double &ay, double &az) {
+  const double qx = wg_div((double)(o.mx * x), o.dx, o.rx), qy = wg_div((double)(o.my * y), o.dy, o.ry);
+  const double q3 = wg_div(o.again == 1 ? qx : qy, 3.0, 1.0 / 3.0);
+  ax = o.again == 1 ? q3 : qx;
+  ay = o.again == 2 ? q3 : qy;
+  az = o.z;
+}
+
+// worldgen.py:27-48 once `start` and the water / mountain octaves (v[0..3]) are known: the next phase.
+CR_DEV int wg_water_mountain(const Geom &g, uint32_t world_seed, int x, int y, WgTile &T, int c, double start,
+                             int &result) {
+  const double *v = T.v[c];
+  double water = (0 + 1 * v[0]) + 0.15 * v[1];  // {15: 1, 5: 0.15}, unnormalised
+  water = water + 0.1;
+  water -= 2 * start;
+  double mountain = (0 + 1 * v[2]) + 0.3 * v[3];  // {15: 1, 5: 0.3}
+  mountain /= (1 + 0.3);
+  mountain -= 4 * start + 0.3 * water;
+  T.water[c] = water; T.mountain[c] = mountain;
+  if (mountain > 0.15)  // caves need `simplex(x, y, 6, 7) > 0.15 and mountain > 0.3` (worldgen.py:40)
+    return mountain > 0.3 ? WP_CAVE : wg_enter_tunnel(g, world_seed, x, y, mountain, T, c);
+  if (0.25 < water && water <= 0.35) return WP_SAND;
+  if (0.3 < water) { result = M_WATER; return WP_DONE; }
+  return wg_enter_tree(g, world_seed, x, y);
 }
 
 // The reference's branch structure for one cell once the octaves of its phase are in v[].
@@ -233,25 +283,10 @@ CR_DEV void wg_combine(const Geom &g, uint32_t world_seed, int x, int y, WgTile 
     case WP_START: {
       int ddx = x - g.W / 2, ddy = y - g.H / 2;  // player at the centre, env.py:71
       double start = 4 - sqrt((double)(ddx * ddx + ddy * ddy));
-      start += 2 * v[0];
+      start += 2 * T.start[c];  // the start octave (slot 4)
       start = 1 / (1 + exp(-start));
       T.start[c] = start;
-      phase = start > 0.5 ? WP_DONE : WP_WM;  // grass
-    } break;
-    case WP_WM: {
-      const double start = T.start[c];
-      double water = (0 + 1 * v[0]) + 0.15 * v[1];  // {15: 1, 5: 0.15}, unnormalised
-      water = water + 0.1;
-      water -= 2 * start;
-      double mountain = (0 + 1 * v[2]) + 0.3 * v[3];  // {15: 1, 5: 0.3}
-      mountain /= (1 + 0.3);
-      mountain -= 4 * start + 0.3 * water;
-      T.water[c] = water; T.mountain[c] = mountain;
-      if (mountain > 0.15)  // caves need `simplex(x, y, 6, 7) > 0.15 and mountain > 0.3` (worldgen.py:40)
-        phase = mountain > 0.3 ? WP_CAVE : wg_enter_tunnel(g, world_seed, x, y, mountain, T, c);
-      else if (0.25 < water && water <= 0.35) phase = WP_SAND;
-      else if (0.3 < water) { result = M_WATER; phase = WP_DONE; }
-      else phase = wg_enter_tree(g, world_seed, x, y);
+      phase = start > 0.5 ? WP_DONE : wg_water_mountain(g, world_seed, x, y, T, c, start, result);  // DONE: grass
     } break;
     case WP_CAVE:  // mountain > 0.3 here
       if (v[0] > 0.15) { result = M_PATH; phase = WP_DONE; }
@@ -294,9 +329,9 @@ CR_DEV void wg_combine(const Geom &g, uint32_t world_seed, int x, int y, WgTile 
 CR_DEV void wg_material_tile(const Geom &g, const NoiseTables &t, uint32_t world_seed, uint8_t *out,
                              int cell0, int ncell, int tid, int nthreads, WgTile &T) {
   for (int c = tid; c < ncell; c += nthreads) T.phase[c] = WP_START;
-  for (int i = tid; i < WG_N_OCTAVES; i += nthreads) T.oct[i] = wg_octave_code(i);
+  for (int i = tid; i < WG_N_OCTAVES; i += nthreads) T.oct[i] = wg_octave(wg_octave_code(i));
   cr_syncblock();
-  for (int round = 0; round < 5; ++round) {
+  for (int round = 0; round < WG_ROUNDS; ++round) {
     if (tid == 0) T.n_items = 0;
     cr_syncblock();
     for (int c = tid; c < ncell; c += nthreads) {
@@ -304,18 +339,20 @@ CR_DEV void wg_material_tile(const Geom &g, const NoiseTables &t, uint32_t world
       if (phase == WP_DONE) continue;
       const unsigned slots = wg_phase_slots(phase, T.need[c]);
       int at = cr_atomic_add_shared(&T.n_items, cr_popc(slots));
-      for (int s2 = 0; s2 < 4; ++s2)
-        if ((slots >> s2) & 1u) T.items[at++] = (uint16_t)(c * 4 + s2);
+      for (int s2 = 0; s2 < WG_SLOTS; ++s2)
+        if ((slots >> s2) & 1u) T.items[at++] = (uint16_t)(c * 8 + s2);
     }
     cr_syncblock();
     const int n = T.n_items;
     if (n == 0) break;  // uniform
     for (int it = tid; it < n; it += nthreads) {
-      const int c = T.items[it] >> 2, slot = T.items[it] & 3;
+      const int c = T.items[it] >> 3, slot = T.items[it] & 7;
       const int cell = cell0 + c, x = cell / g.H, y = cell - x * g.H;
       double ax, ay, az;
       wg_octave_args(T.oct[T.phase[c] * 4 + slot], x, y, ax, ay, az);
-      T.v[c][slot] = noise3(t, ax, ay, az);
+      const double value = noise3(t, ax, ay, az);
+      if (slot < 4) T.v[c][slot] = value;
+      else T.start[c] = value;
     }
     cr_syncblock();
     for (int c = tid; c < ncell; c += nthreads) {
